@@ -16,8 +16,11 @@ gradient all-reduce (N>1), clip + AdamW + EMA teacher.  Synthetic N(0,1) crops, 
 `parity` : one step of the bench model (same weights, drop-path off) on the first 4 images of the bench batch against
            the autocast-emulating oracle on the host: loss delta and logit errors.
 `cpu_baseline` / `--impl reference`: the reference's OWN DINOv2 method class (unmodified source from baseline/_ref or
-           /root/reference, absent third-party packages stubbed: oracle/ref_full.py) on the host cores;
+           $LIGHTLY_TRAIN_SRC, absent third-party packages stubbed: oracle/ref_full.py) on the host cores;
 `gpu_torch_baseline`: those same reference modules on the B200 under torch.autocast(bf16), eager -- "the kernel to beat".
+`--dump-outputs DIR`: after the timed steps, what the last of them handed back (loss and its terms) and left in the model
+           (a fixed, seeded sample of the student / teacher weights, the loss centers) as DIR/<name>.npy, so that two
+           builds can be compared output for output on identical inputs.
 """
 from __future__ import annotations
 
@@ -281,6 +284,32 @@ def run_reference_arm(args) -> None:
     print(json.dumps(line), flush=True)
 
 
+# --------------------------------------------------------------------------------------------- output dump
+DUMP_SAMPLE = 1 << 20  # elements kept of each large tensor (4 MB in float32)
+
+
+def _sample(x: "torch.Tensor", seed: int) -> "torch.Tensor":
+    """A fixed, seeded sample of DUMP_SAMPLE elements of a flat tensor (all of it when smaller)."""
+    x = x.detach().flatten()
+    if x.numel() <= DUMP_SAMPLE:
+        return x
+    idx = torch.randint(0, x.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(seed)).to(x.device)
+    return x[idx]
+
+
+def dump_outputs(out_dir: str, res, tensors: dict) -> None:
+    """Write the step result (loss and every log_dict term) and `tensors` (sampled) as float32 .npy files."""
+    import numpy as np
+
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    arrays = {"loss": res.loss}
+    arrays.update({k.split("/")[-1]: v for k, v in res.log_dict.items()})
+    arrays.update({k: _sample(v, seed=i) for i, (k, v) in enumerate(tensors.items())})
+    for k, v in arrays.items():
+        np.save(d / f"{k}.npy", torch.as_tensor(v).detach().float().cpu().numpy())
+
+
 # --------------------------------------------------------------------------------------------- parity of the bench model
 def bench_parity(method, cfg: dict, views_dev, dev) -> dict:
     """One step (drop-path off, eager) of a copy of the bench model on the first 4 images of the bench batch vs the
@@ -394,6 +423,8 @@ def run_distill(args) -> None:
         e1.record()
         barrier()
     launches = _lib.LAUNCHES - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, {"student_params": torch.cat([p.detach().flatten() for p in params])})
     t = torch.tensor([e0.elapsed_time(e1) / K], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -464,7 +495,11 @@ def main() -> None:
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--eager", action="store_true", help="launch every kernel from the host instead of CUDA-graph replay")
     ap.add_argument("--gemm-profile", default="", help="write the per-shape GEMM timing table of one step to this file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (float32, large tensors sampled)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -533,6 +568,9 @@ def main() -> None:
     launches = _lib.LAUNCHES - l0
     ms = e0.elapsed_time(e1) / K
     loss_val = float(res.loss)
+    if args.dump_outputs and rank == 0:  # before the e2e steps below overwrite the graph's outputs and the weights
+        dump_outputs(args.dump_outputs, res, {"student_params": method.s_arena.fp32, "teacher_params": method.t_arena.fp32,
+                                              "dino_center": method.dino_loss.center, "ibot_center": method.ibot_loss.center})
     t = torch.tensor([ms], device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)

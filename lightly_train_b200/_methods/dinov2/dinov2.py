@@ -463,6 +463,9 @@ class DINOv2(nn.Module):
 
     def training_step_impl(self, batch: Dict[str, Any], batch_idx: int = 0) -> TrainingStepResult:
         """Loss evaluation + explicit backward (gradients land in the arena / `param.grad`). Eager launch schedule."""
+        # the kernels take raw device pointers: a model built in host memory fails here, before any launch (with a GPU
+        # present such a launch would fault asynchronously and leave the CUDA context unusable)
+        ops._req_cuda(self.s_arena.fp32)
         a = self.method_args
         dev = self.device_
         teacher_temp = linear_warmup_schedule(self.trainer.global_step, a.teacher_temp_warmup_steps,
@@ -1009,6 +1012,7 @@ class DINOv2(nn.Module):
 
     def train_step(self, batch: Dict[str, Any]) -> TrainingStepResult:
         """One full optimisation step: what Lightning's fit loop does around training_step (SURVEY.md 3.1)."""
+        ops._req_cuda(self.s_arena.fp32)
         if self._graph_ok():
             res = self._graphed_step(batch)
         else:

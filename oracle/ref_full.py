@@ -1,8 +1,8 @@
 """TEST / BENCH INFRASTRUCTURE -- never imported by the product package (lightly_train_b200/).
 
 Runs the reference's OWN method class (`lightly_train._methods.dinov2.dinov2.DINOv2`, unmodified source) without its
-absent third-party packages.  The reference source is taken from /root/reference/src (build container) or from
-`baseline/_ref` (the `pip install --no-deps --target baseline/_ref` copy that travels to the GPU box).  Its
+absent third-party packages.  The reference source is taken from the directory named by $LIGHTLY_TRAIN_SRC (the `src`
+directory of a lightly-train checkout) or from `baseline/_ref` (a `pip install --no-deps --target baseline/_ref` copy).  Its
 dependencies that are NOT in this image -- pytorch_lightning, lightly, omegaconf, albumentations, lightning_utilities,
 ... -- are replaced by stubs:
 
@@ -34,7 +34,7 @@ import torch
 from torch import Tensor, nn
 
 ROOT = Path(__file__).resolve().parents[1]
-CANDIDATES = [Path("/root/reference/src"), ROOT / "baseline" / "_ref"]
+CANDIDATES = [Path(p) for p in (os.environ.get("LIGHTLY_TRAIN_SRC"),) if p] + [ROOT / "baseline" / "_ref"]
 
 _STUB_ROOTS = ("pytorch_lightning", "lightly", "lightning_utilities", "omegaconf", "albumentations", "lightning_fabric",
                "wandb", "mlflow", "tensorboard", "cv2", "pydicom", "timm", "xformers", "rfdetr", "ultralytics", "super_gradients",
@@ -43,8 +43,11 @@ _STUB_ROOTS = ("pytorch_lightning", "lightly", "lightning_utilities", "omegaconf
 
 def source_root() -> Optional[Path]:
     for c in CANDIDATES:
-        if (c / "lightly_train" / "_methods" / "dinov2" / "dinov2.py").is_file():
-            return c
+        try:
+            if (c / "lightly_train" / "_methods" / "dinov2" / "dinov2.py").is_file():
+                return c
+        except OSError:  # e.g. a directory this user may not read
+            pass
     return None
 
 
@@ -281,7 +284,7 @@ def install() -> None:
         return
     src = source_root()
     if src is None:
-        raise RuntimeError("reference source not found (neither /root/reference/src nor baseline/_ref)")
+        raise RuntimeError("reference source not found (set LIGHTLY_TRAIN_SRC or install a copy into baseline/_ref)")
     os.environ["XFORMERS_DISABLED"] = "1"
     for name in list(sys.modules):
         if name.split(".")[0] in ("lightly_train", "lightning_utilities"):

@@ -1,12 +1,12 @@
-"""Import the reference's own hot-path modules in place from /root/reference (build container only).
+"""Import the reference's own hot-path modules in place from a lightly-train source tree ($LIGHTLY_TRAIN_SRC, the
+checkout's `src` directory).
 
 `import lightly_train` itself fails here (its __init__ pulls pytorch_lightning / albumentations / omegaconf /
 lightly, none installed).  Registering an empty namespace package whose __path__ is the reference source
 directory skips that __init__, and a 5-line stub of lightning_utilities.core.imports.RequirementCache (used at
 vision_transformer.py:24,43) is enough for the arithmetic modules to import unmodified:
   _methods.dinov2.{dinov2_loss,dinov2_head,utils,scheduler}, _models.dinov2_vit.dinov2_vit_src.*, _torch_helpers.
-/root/reference does not exist on the GPU box: nothing under `-m gpu`, smoke() or bench.py may call this.
-Used by tools/make_golden.py (fixture generation) and tests/test_oracle_vs_reference.py (skipped when absent).
+Only the fixture generators under tools/ use this; the tests read what they wrote under tests/golden/.
 """
 from __future__ import annotations
 
@@ -15,18 +15,21 @@ import sys
 import types
 from pathlib import Path
 
-REF_SRC = Path("/root/reference/src/lightly_train")
+REF_SRC = Path(os.environ.get("LIGHTLY_TRAIN_SRC", "")) / "lightly_train"
 
 
 def available() -> bool:
-    return REF_SRC.is_dir()
+    try:
+        return "LIGHTLY_TRAIN_SRC" in os.environ and REF_SRC.is_dir()
+    except OSError:
+        return False
 
 
 def install() -> None:
     if "lightly_train" in sys.modules:
         return
     if not available():
-        raise RuntimeError("/root/reference is not present (it never is on the GPU box)")
+        raise RuntimeError("set LIGHTLY_TRAIN_SRC to the src directory of a lightly-train checkout")
     os.environ["XFORMERS_DISABLED"] = "1"
     pkg = types.ModuleType("lightly_train")
     pkg.__path__ = [str(REF_SRC)]  # namespace-style: skips lightly_train/__init__.py

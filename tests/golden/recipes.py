@@ -83,6 +83,14 @@ def _fill(name: str, shape: Tuple[int, ...], g: torch.Generator) -> Tensor:
     return r * (0.7 / fan_in ** 0.5)
 
 
+def sample_index(numel: int, n: int) -> Tensor:
+    """n distinct flat indices spread over a tensor of `numel` elements (all of them when numel <= n): where a fixture
+    would otherwise hold a whole gradient or weight tensor, it holds these elements only."""
+    if numel <= n:
+        return torch.arange(numel)
+    return (torch.arange(n, dtype=torch.int64) * 2654435761 + 97) % numel  # prime stride: distinct for numel < 2654435761
+
+
 def det_vit_state(cfg: O.ViTConfig, seed: int) -> Dict[str, Tensor]:
     g = torch.Generator().manual_seed(seed)
     return {k: _fill(k, s, g) for k, s in vit_param_shapes(cfg).items()}
@@ -199,6 +207,24 @@ def det_dinov3_state(cfg, seed: int) -> Dict[str, Tensor]:
     for k, shp in dinov3_param_shapes(cfg).items():
         out[k] = _fill("register_tokens" if k == "storage_tokens" else k, shp, g)
     return out
+
+
+# ---------------------------------------------------------------- DistillationV3 step (DINOv3 teacher -> ResNet-18 student)
+DISTILL_TEACHER_KW = dict(img_size=224, patch_size=16, embed_dim=128, depth=2, num_heads=2, ffn_ratio=4.0, layerscale_init=1e-5,
+                          norm_layer="layernormbf16", n_storage_tokens=4, mask_k_bias=True, pos_embed_rope_dtype="fp32")
+
+
+def det_fill_(module: torch.nn.Module, seed: int) -> None:
+    """Deterministic weights for a module whose parameter names are the same on both sides (biases small, matrices
+    0.7 / sqrt(fan_in))."""
+    g = torch.Generator().manual_seed(seed)
+    with torch.no_grad():
+        for k, p in sorted(module.named_parameters()):
+            p.copy_(_fill(k, tuple(p.shape), g))
+
+
+def distill_step_input() -> Tensor:
+    return torch.randn(4, 3, 224, 224, generator=torch.Generator().manual_seed(403))
 
 
 def dinov3_case_inputs() -> Tuple[Tensor, Tensor]:

@@ -1,6 +1,7 @@
 """BASELINE.json configurations as parity cases, and helpers that drive the reference's OWN method class (through
-oracle/ref_full.py: reference source from /root/reference or baseline/_ref, absent third-party packages stubbed) next to
-the oracle and the CUDA mirror on identical weights, crops and masks.  Test infrastructure only."""
+oracle/ref_full.py: reference source from $LIGHTLY_TRAIN_SRC or baseline/_ref, absent third-party packages stubbed) next
+to the oracle and the CUDA mirror on identical weights, crops and masks.  The tests compare with what
+tools/make_method_golden.py stored from such runs under tests/golden/; only that tool needs the reference."""
 from __future__ import annotations
 
 import random
@@ -110,6 +111,24 @@ def oracle_state(ref_state: Dict[str, Tensor], separate: bool) -> Tuple[Dict[str
                 out[who]["ibot_head." + k[len(f"{who}_head.ibot_head."):]] = v.detach().clone().float()
     centers = {"dino": ref_state["dino_loss.center"].clone(), "ibot": ref_state["ibot_loss.center"].clone()}
     return out["student"], out["teacher"], centers
+
+
+def load_oracle_state(m, student: Dict[str, Tensor], teacher: Dict[str, Tensor], centers: Dict[str, Tensor]) -> None:
+    """Inverse of `oracle_state`: write flat oracle weights into a method's state_dict (reference or mirror naming); a
+    shared iBOT head takes the DINO head's weights."""
+    sd = m.state_dict()
+    new = {}
+    for who, flat in (("student", student), ("teacher", teacher)):
+        for k, v in flat.items():
+            if k.startswith("backbone."):
+                new[f"{who}_embedding_model.wrapped_model._model." + k[len("backbone."):]] = v
+            else:
+                new[f"{who}_head." + k] = v
+                if k.startswith("dino_head.") and f"{who}_head.ibot_{k[len('dino_'):]}" in sd and "ibot_head." + k[len("dino_head."):] not in flat:
+                    new[f"{who}_head.ibot_{k[len('dino_'):]}"] = v
+    new["dino_loss.center"], new["ibot_loss.center"] = centers["dino"], centers["ibot"]
+    assert set(new) == set(sd), set(new) ^ set(sd)
+    m.load_state_dict({k: new[k].reshape(sd[k].shape) for k in sd}, strict=True)
 
 
 def oracle_cfg(case: Case) -> O.StepConfig:

@@ -1,8 +1,7 @@
 """-m gpu: the distillation path (BASELINE cfg4; SURVEY 8a rows a16 / a17) -- RoPE kernel, fused KL kernels, the DINOv3
 teacher forward on the B200 kernels against the oracle and the reference-generated fixtures, and the whole DistillationV3
-step against the reference's OWN method class (through oracle/ref_full.py) on identical weights, inputs and mixup draws."""
-import copy
-
+step against the reference's OWN method class (stored from a run through oracle/ref_full.py) on identical weights,
+inputs and mixup draws."""
 import pytest
 import torch
 import torch.nn.functional as F
@@ -19,7 +18,6 @@ from lightly_train_b200._models.dinov3_vit import DinoV3VisionTransformer, DINOv
 from lightly_train_b200._models.torchvision_resnet import EmbeddingModel, ResNetModelWrapper  # noqa: E402
 from oracle import dinov3_oracle as D3  # noqa: E402
 from oracle import distillationv3_oracle as DO  # noqa: E402
-from oracle import ref_full  # noqa: E402
 from tests.golden import recipes as R  # noqa: E402
 
 dev = "cuda"
@@ -91,62 +89,45 @@ def test_dinov3_teacher_forward_parity(golden_dir):
     assert {"rope_embed.periods", "blocks.0.attn.qkv.bias_mask", "storage_tokens", "cls_token", "mask_token"} <= names
 
 
-@pytest.mark.skipif(not ref_full.available(), reason="reference copy (baseline/_ref) not on this box")
-def test_distillation_step_matches_reference_method():
+def test_distillation_step_matches_reference_method(golden_dir):
+    """Two training_step_impl calls and the backward of the second against the reference's own DistillationV3 (stored by
+    tools/make_method_golden.py): same teacher and projection-head weights (recipes), same ResNet-18 initialisation
+    (torch.manual_seed(0)), same input and mixup seeds.  Gradients are compared at the stored elements."""
     import torchvision
 
-    ref_full.install()
-    from lightly_train._methods.distillationv3.distillationv3 import DistillationV3 as RefMethod  # type: ignore
-    from lightly_train._methods.distillationv3.distillationv3 import DistillationV3AdamWArgs, DistillationV3Args as RefArgs  # type: ignore
-    from lightly_train._models.dinov3.dinov3_src.models import vision_transformer as v3  # type: ignore
-    from lightly_train._models.dinov3.dinov3_vit import DINOv3ViTModelWrapper as RefTeacherWrapper  # type: ignore
-    from lightly_train._models.embedding_model import EmbeddingModel as RefEmbedding  # type: ignore
-    from lightly_train._models.torchvision.resnet import ResNetModelWrapper as RefResNetWrapper  # type: ignore
-
+    ref = torch.load(golden_dir / "distillation_v3_step.pt")
+    tvit = DinoV3VisionTransformer(**R.DISTILL_TEACHER_KW)
+    r = tvit.load_state_dict(R.det_dinov3_state(R.dinov3_tiny_cfg(), seed=15), strict=False)
+    assert not r.unexpected_keys and all(k.endswith("bias_mask") or k == "rope_embed.periods" for k in r.missing_keys), r
     torch.manual_seed(0)
-    kw = dict(img_size=224, patch_size=16, embed_dim=128, depth=2, num_heads=2, ffn_ratio=4.0, layerscale_init=1e-5,
-              norm_layer="layernormbf16", n_storage_tokens=4, mask_k_bias=True, pos_embed_rope_dtype="fp32")
-    rvit = v3.DinoVisionTransformer(**kw)
-    rvit.init_weights()
-    with torch.no_grad():  # O(1) LayerScale so that the blocks matter
-        for n, p in rvit.named_parameters():
-            if n.endswith("gamma"):
-                p.fill_(0.5)
     resnet = torchvision.models.resnet18()
-    rm = RefMethod(RefArgs(queue_size=64, teacher=RefTeacherWrapper(rvit)), DistillationV3AdamWArgs(),
-                   RefEmbedding(wrapped_model=RefResNetWrapper(resnet)), global_batch_size=4, num_input_channels=3)
-    rm.trainer = ref_full._Trainer(10)
-
-    tvit = DinoV3VisionTransformer(**kw)
-    tvit.load_state_dict(rvit.state_dict(), strict=True)
-    student = EmbeddingModel(ResNetModelWrapper(copy.deepcopy(resnet))).to(dev)
+    student = EmbeddingModel(ResNetModelWrapper(resnet)).to(dev)
     mm = DistillationV3(DistillationV3Args(queue_size=64), None, student, 4, 3, teacher_embedding_model=DINOv3ViTModelWrapper(tvit)).to(dev)
-    with torch.no_grad():
-        for n in ("student_projection_head_global", "student_projection_head_local"):
-            getattr(mm, n).load_state_dict(getattr(rm, n).state_dict())
-    x = torch.randn(4, 3, 224, 224)
+    for n in ("student_projection_head_global", "student_projection_head_local"):
+        R.det_fill_(getattr(mm, n), seed=16)
+    x = R.distill_step_input()
     for step in range(2):  # second step: the queue already holds the first batch
-        torch.manual_seed(100 + step)
-        rres = rm.training_step_impl({"views": [x]}, 0)
         torch.manual_seed(100 + step)
         with torch.autocast("cuda", dtype=torch.bfloat16):
             mres = mm.training_step_impl({"views": [x.to(dev)]}, 0)
-        for k in ("train_loss/global_loss", "train_loss/local_loss"):
-            a, b = float(mres.log_dict[k]), float(rres.log_dict[k])
+        want = ref["steps"][step]
+        for k in ("global_loss", "local_loss"):
+            a, b = float(mres.log_dict["train_loss/" + k]), want[k]
             assert abs(a - b) < 2e-2 * max(1.0, abs(b)), (step, k, a, b)  # bf16 autocast student + bf16 teacher vs fp32 reference
-        assert (mm.teacher_queue.cpu() - rm.teacher_queue).abs().max().item() < 3e-2
-    rres.loss.backward()
+        q = torch.zeros_like(mm.teacher_queue, device="cpu")
+        q[:want["queue_head"].shape[0]] = want["queue_head"]  # the rest of the reference queue is still zero
+        assert (mm.teacher_queue.cpu() - q).abs().max().item() < 3e-2
     mres.loss.backward()
-    ga = mm.student_projection_head_global.weight.grad.float().cpu()
-    gb = rm.student_projection_head_global.weight.grad
-    assert ((ga - gb).norm() / gb.norm()).item() < 0.1
+    res = mm.student_embedding_model.wrapped_model.get_model()
+    got = {"head_global": mm.student_projection_head_global.weight.grad, "layer4.1.conv2": res.layer4[1].conv2.weight.grad,
+           "conv1": res.conv1.weight.grad}
+    got = {k: v.float().cpu().flatten()[R.sample_index(v.numel(), ref["grads"][k]["sample"].numel())] for k, v in got.items()}
+    gb = ref["grads"]["head_global"]["sample"]
+    assert ((got["head_global"] - gb).norm() / gb.norm()).item() < 0.1
     # deep in the student (bf16 autocast convs + BatchNorm over 4 images vs the fp32 reference): direction, not digits
-    ga = mm.student_embedding_model.wrapped_model.get_model().layer4[1].conv2.weight.grad.float().cpu().flatten()
-    gb = rm.student_embedding_model.wrapped_model.get_model().layer4[1].conv2.weight.grad.flatten()
-    assert torch.nn.functional.cosine_similarity(ga, gb, dim=0).item() > 0.9
-    ga = mm.student_embedding_model.wrapped_model.get_model().conv1.weight.grad.float().cpu().flatten()
-    gb = rm.student_embedding_model.wrapped_model.get_model().conv1.weight.grad.flatten()
-    assert torch.nn.functional.cosine_similarity(ga, gb, dim=0).item() > 0.6
+    cos = torch.nn.functional.cosine_similarity
+    assert cos(got["layer4.1.conv2"], ref["grads"]["layer4.1.conv2"]["sample"], dim=0).item() > 0.9
+    assert cos(got["conv1"], ref["grads"]["conv1"]["sample"], dim=0).item() > 0.6
 
 
 def test_sibling_distillation_losses():

@@ -127,22 +127,20 @@ def test_state_dict_names_and_shapes_match_the_reference_modules(golden_dir):
         assert got == ref[name], (name, set(got) ^ set(ref[name]))
 
 
-def test_chunked_block_checkpoint_names_load():
-    """Zoo configs with block_chunks > 0 (ViT-L / ViT-g) name their blocks `blocks.{chunk}.{i}.*`; the mirror loads them."""
-    import pytest
-    import torch
-
-    from oracle import ref_full
-    if not ref_full.available():
-        pytest.skip("reference source not present")
-    ref_full.install()
-    from lightly_train._models.dinov2_vit.dinov2_vit_src.models.vision_transformer import DinoVisionTransformer as RefViT  # type: ignore
+def test_chunked_block_checkpoint_names_load(golden_dir):
+    """Zoo configs with block_chunks > 0 (ViT-L / ViT-g) name their blocks `blocks.{chunk}.{i}.*`; the mirror loads them.
+    The checkpoint has the layout of the reference's own DinoVisionTransformer(block_chunks=2) (names and shapes stored by
+    tools/make_method_golden.py) and seeded random values."""
+    import json
 
     from lightly_train_b200._models.dinov2_vit import DinoVisionTransformer
 
-    r = RefViT(embed_dim=128, depth=4, num_heads=2, block_chunks=2, init_values=1e-5)
+    layout = json.loads((golden_dir / "method_boundary.json").read_text())["chunked_vit_state_dict"]
+    g = torch.Generator().manual_seed(3)
+    r = {k: torch.randn(shape, generator=g) for k, shape in layout}
+    assert "blocks.1.3.attn.qkv.weight" in r
     m = DinoVisionTransformer(embed_dim=128, depth=4, num_heads=2, init_values=1e-5, device="cpu")
-    res = m.load_state_dict(r.state_dict(), strict=True)
+    res = m.load_state_dict(r, strict=True)
     assert not res.missing_keys and not res.unexpected_keys
-    assert torch.equal(m.state_dict()["blocks.3.attn.qkv.weight"], r.state_dict()["blocks.1.3.attn.qkv.weight"])
+    assert torch.equal(m.state_dict()["blocks.3.attn.qkv.weight"], r["blocks.1.3.attn.qkv.weight"])
     assert not m.arena.bf16_valid

@@ -16,7 +16,6 @@ from lightly_train_b200._methods.dinov2.dinov2 import DINOv2, DINOv2AdamWViTArgs
 from lightly_train_b200._models.dinov2_vit import DinoVisionTransformer  # noqa: E402
 from lightly_train_b200._torch_helpers import update_momentum  # noqa: E402
 from oracle import dinov2_oracle as O  # noqa: E402
-from oracle import ref_full  # noqa: E402
 from tests import ref_cases as RC  # noqa: E402
 from tests.golden import recipes as R  # noqa: E402
 
@@ -147,38 +146,38 @@ def test_checkpoint_resume_is_exact():
     assert d.max().item() < 3 * a.base_lr and d.mean().item() < 2e-5 and (d > 1e-5).float().mean().item() < 0.15
 
 
-@pytest.mark.skipif(not ref_full.available(), reason="reference copy (baseline/_ref) not on this box")
-def test_checkpoint_round_trip_into_reference_modules():
-    """1 optimisation step on CUDA -> state_dict() -> load_state_dict(strict=True) into the reference's own DINOv2 method
-    -> the reference ViT + head forward (fp32, host) reproduces the CUDA teacher/student features."""
+def test_checkpoint_round_trip_into_reference_modules(golden_dir):
+    """1 optimisation step on CUDA -> state_dict() in exactly the reference DINOv2 method's checkpoint layout (names, order
+    and shapes stored from the reference's own class by tools/make_method_golden.py, so its load_state_dict(strict=True)
+    takes it) -> the fp32 ViT forward on those weights (the oracle, pinned against the reference modules by
+    tests/test_oracle_goldens.py) reproduces the CUDA teacher/student features."""
+    import json
+
     case = RC.TINY
-    ref, _, _ = RC.build_reference(case)
+    cfg = RC.oracle_cfg(case)
+    st = R.det_step_state(cfg, seed=41)
+    mk = {k: v for k, v in case.vit.items() if k != "block_chunks"}
     m = DINOv2(DINOv2Args(**dict(dict(warmup_steps=2, student_freeze_last_layer_steps=1), **case.method)), DINOv2AdamWViTArgs(),
-               ref.teacher_embedding_model, case.batch, 3, max_steps=100, device=dev)
-    m.load_state_dict(ref.state_dict(), strict=True)
+               mk, case.batch, 3, max_steps=100, device=dev)
+    RC.load_oracle_state(m, st["student"], st["teacher"], st["centers"])
     views = RC.make_views(case)
     random.seed(3)
     m.train_step({"views": [v.to(dev) for v in views]})
     m.dino_loss.apply_center_update(); m.ibot_loss.apply_center_update()
     sd = {k: v.detach().cpu() for k, v in m.state_dict().items()}
-    res = ref.load_state_dict(sd, strict=True)
-    assert not res.missing_keys and not res.unexpected_keys
+    layout = json.loads((golden_dir / "method_boundary.json").read_text())["tiny_method_state_dict"]
+    assert [[k, list(v.shape)] for k, v in sd.items()] == layout
+    student, teacher, _ = RC.oracle_state(sd, cfg.ibot_separate_head)
     x = views[0]
     with torch.no_grad():
-        for side in ("teacher", "student"):
-            emb = getattr(ref, f"{side}_embedding_model")
-            want = emb.wrapped_model.get_model().forward_features(x)["x_norm_clstoken"]
+        for side, w in (("teacher", teacher), ("student", student)):
+            want = O.vit_forward_features(O._sub(w, "backbone."), cfg.vit, x)["cls"]
             got = getattr(m, f"{side}_embedding_model").wrapped_model.get_model().forward_features(x.to(dev))["x_norm_clstoken"]
             assert (got.float().cpu() - want).abs().max().item() < 5e-2, side  # bf16 GEMMs vs fp32, O(1) features
             assert (got.float().cpu() - want).abs().mean().item() < 5e-3, side
     # the step really moved the student away from the teacher-initialised weights
     assert (sd["student_embedding_model.wrapped_model._model.blocks.0.attn.qkv.weight"]
-            - ref_full_state_before(case)).abs().max().item() > 0
-
-
-def ref_full_state_before(case):
-    ref0, _, _ = RC.build_reference(case)
-    return ref0.state_dict()["student_embedding_model.wrapped_model._model.blocks.0.attn.qkv.weight"]
+            - st["student"]["backbone.blocks.0.attn.qkv.weight"]).abs().max().item() > 0
 
 
 def test_stochastic_depth_rng_paths():

@@ -3,10 +3,10 @@ depths, head sizes, crop counts and token counts with the batch reduced so that 
 against
   * the autocast-emulating oracle (= the numerics of the reference's CUDA bf16-autocast path): 1e-3 on every loss term,
     mean |logit error| < 1e-3, max < one bf16 ulp of an O(1) logit (7.8e-3);
-  * the reference's OWN method class run in fp32 on the host cores (oracle/ref_full.py over baseline/_ref), when that
-    copy travelled to this box: 5e-3 on the loss terms (bf16-vs-fp32), gradients norm-wise.
-The mirror is built from the reference's embedding model (reference ctor) and loads the reference method's state_dict
-with strict=True, so checkpoint-name compatibility is exercised at the real sizes too.
+  * the reference's OWN method class run in fp32 on the host cores (oracle/ref_full.py, by tools/make_method_golden.py,
+    which stored its loss terms and, per gradient tensor, the norm and the elements at `recipes.sample_index` under
+    tests/golden/parity_*.pt): 5e-3 on the loss terms (bf16-vs-fp32), gradients norm-wise against the fp32 oracle's full
+    gradients, which must first reproduce the stored ones.
 """
 import dataclasses
 import random
@@ -21,23 +21,11 @@ if not torch.cuda.is_available():
 
 from lightly_train_b200._methods.dinov2.dinov2 import DINOv2, DINOv2AdamWViTArgs, DINOv2Args  # noqa: E402
 from oracle import dinov2_oracle as O  # noqa: E402
-from oracle import ref_full  # noqa: E402
 from tests import ref_cases as RC  # noqa: E402
+from tests.golden import recipes as R  # noqa: E402
 
 dev = "cuda"
 RESULTS = {}
-
-
-def _mirror_from_reference(case: RC.Case, ref) -> DINOv2:
-    margs = dict(warmup_steps=2, student_freeze_last_layer_steps=1, teacher_temp_start=0.05, teacher_temp_end=0.05)
-    margs.update(case.method)
-    m = DINOv2(DINOv2Args(**margs), DINOv2AdamWViTArgs(), ref.teacher_embedding_model, case.batch, 3, max_steps=100, device=dev)
-    missing = m.load_state_dict(ref.state_dict(), strict=True)
-    assert not missing.missing_keys and not missing.unexpected_keys
-    assert not m.s_arena.bf16_valid and not m.t_arena.bf16_valid  # load_state_dict post-hook
-    if case.checkpointing:
-        m.student_embedding_model.wrapped_model.set_activation_checkpointing(True)
-    return m
 
 
 def _mirror_from_state(case: RC.Case, student, teacher, centers) -> DINOv2:
@@ -45,15 +33,15 @@ def _mirror_from_state(case: RC.Case, student, teacher, centers) -> DINOv2:
     margs.update(case.method)
     mk = {k: v for k, v in case.vit.items() if k not in ("block_chunks",)}
     m = DINOv2(DINOv2Args(**margs), DINOv2AdamWViTArgs(), mk, case.batch, 3, max_steps=100, device=dev)
-    m.s_arena.load_from(student)
-    m.t_arena.load_from(teacher)
-    m.dino_loss.center.copy_(centers["dino"])
-    m.ibot_loss.center.copy_(centers["ibot"])
+    RC.load_oracle_state(m, student, teacher, centers)  # load_state_dict(strict=True) in the reference's checkpoint names
+    assert not m.s_arena.bf16_valid and not m.t_arena.bf16_valid  # load_state_dict post-hook
+    if case.checkpointing:
+        m.student_embedding_model.wrapped_model.set_activation_checkpointing(True)
     return m
 
 
 @pytest.mark.parametrize("case", [RC.CFG1, RC.CFG2, RC.CFG3, RC.CFG5], ids=lambda c: c.name)
-def test_step_parity_at_baseline_dims(case):
+def test_step_parity_at_baseline_dims(case, golden_dir):
     torch.set_num_threads(min(32, torch.get_num_threads() if torch.get_num_threads() > 1 else 32))
     # KoLeo enters the loss with weight 0 here (its VALUE is still computed, logged and compared): -log of the nearest-
     # neighbour distance between a handful of nearly identical cls features is so ill-conditioned that bf16 rounding alone
@@ -61,19 +49,11 @@ def test_step_parity_at_baseline_dims(case):
     # tensor 0.46 with the term, 0.013 without), which would drown the comparison of everything else; the term is
     # third-party and unpinned anyway (DESIGN.md section 4).  Its kernel gradient is checked in tests/test_kernels_gpu.py.
     case = dataclasses.replace(case, method=dict(case.method, koleo_loss_weight=0.0))
-    have_ref = ref_full.available()
     views = RC.make_views(case)
     cfg = dataclasses.replace(RC.oracle_cfg(case), koleo_loss_weight=0.0)
-    if have_ref:
-        ref, _, _ = RC.build_reference(case)
-        ref_sd = {k: v.detach().clone() for k, v in ref.state_dict().items()}
-        student, teacher, centers = RC.oracle_state(ref_sd, cfg.ibot_separate_head)
-        m = _mirror_from_reference(case, ref)
-    else:  # same deterministic construction without the reference classes
-        from tests.golden import recipes as R
-        st = R.det_step_state(cfg, seed=41)
-        student, teacher, centers = st["student"], st["teacher"], st["centers"]
-        m = _mirror_from_state(case, student, teacher, centers)
+    st = R.det_step_state(cfg, seed=41)
+    student, teacher, centers = st["student"], st["teacher"], st["centers"]
+    m = _mirror_from_state(case, student, teacher, centers)
     mk = RC.masks_for(case, 11)
 
     # ---- CUDA step (masks drawn by the mirror itself from the same python RNG stream as the reference)
@@ -110,33 +90,44 @@ def test_step_parity_at_baseline_dims(case):
         assert rec[side]["mean"] < 1e-3, rec
         assert rec[side]["max"] < 1.6e-2, rec  # two bf16 ulps of a logit in [1, 2): rounding-boundary flips only
 
-    # ---- the reference's own method class, fp32 on the host cores
-    if have_ref:
-        terms, grads = RC.reference_losses(ref, views, mask_seed=11)
-        rec["reference_fp32"] = terms
-        for k in got:
-            tol = 5e-2 if k == "koleo_loss" else 5e-3
-            assert abs(got[k] - terms[k]) < tol * max(1.0, abs(terms[k])), (k, got[k], terms[k])
-        # Gradients vs the reference's fp32 autograd, norm-wise per tensor.  The yardstick is the autocast-emulating oracle's own
-        # distance from the same fp32 gradients (bf16 rounding of a correct step): the CUDA path may not be further away than
-        # that (x1.5 + 0.03), and never further than 8e-2.
-        worst = ("", 0.0, 0.0)
-        errs, oerrs = [], []
-        for k in student:
-            name = ("student_embedding_model.wrapped_model._model." + k[len("backbone."):]) if k.startswith("backbone.") else "student_head." + k
-            gref = grads.get(name)
-            if gref is None or gref.norm().item() < 1e-9:
-                continue
-            e = (m.s_arena.g(k).float().cpu() - gref).norm().item() / gref.norm().item()
-            eo = (ostudent[k].grad - gref).norm().item() / gref.norm().item()
-            errs.append(e); oerrs.append(eo)
-            if e - 1.5 * eo > worst[1] - 1.5 * worst[2]:
-                worst = (k, e, eo)
-        rec["grad_rel_err"] = {"worst_excess": worst, "median": sorted(errs)[len(errs) // 2], "max": max(errs),
-                               "autocast_oracle_median": sorted(oerrs)[len(oerrs) // 2], "autocast_oracle_max": max(oerrs)}
-        assert worst[1] < 1.5 * worst[2] + 0.03, (worst, rec["grad_rel_err"])
-        assert rec["grad_rel_err"]["max"] < 8e-2, rec["grad_rel_err"]
-        assert rec["grad_rel_err"]["median"] < 1.5 * rec["grad_rel_err"]["autocast_oracle_median"] + 0.01, rec["grad_rel_err"]
+    # ---- the reference's own method class, fp32 on the host cores (stored)
+    ref = torch.load(golden_dir / f"parity_{case.name.split('_')[0]}.pt")
+    terms = ref["terms"]
+    rec["reference_fp32"] = terms
+    for k in got:
+        tol = 5e-2 if k == "koleo_loss" else 5e-3
+        assert abs(got[k] - terms[k]) < tol * max(1.0, abs(terms[k])), (k, got[k], terms[k])
+    # The reference's fp32 gradients in full: the oracle without autocast, first pinned to what is stored from the
+    # reference (every gradient norm and the stored elements of every tensor, 1e-4).
+    fstudent = {k: v.clone().requires_grad_(True) for k, v in student.items()}
+    O.training_step(cfg, fstudent, teacher, centers, views, mk["collated_masks"], mk["mask_indices_list"], mk["masks_weight"],
+                    teacher_temp=0.05)["loss"].backward()
+    grads = {}
+    for i, k in enumerate(ref["names"]):
+        g, gnorm, gs = fstudent[k].grad, float(ref["grad_norm"][i]), ref["grad_sample"][i]
+        idx = R.sample_index(g.numel(), gs.numel())
+        assert abs(g.norm().item() - gnorm) <= 1e-4 * gnorm, (k, g.norm().item(), gnorm)
+        assert (g.flatten()[idx] - gs).norm().item() <= 1e-4 * (gs.norm().item() + gnorm * (idx.numel() / g.numel()) ** 0.5), k
+        grads[k] = g
+    # Gradients vs the reference's fp32 autograd, norm-wise per tensor.  The yardstick is the autocast-emulating oracle's own
+    # distance from the same fp32 gradients (bf16 rounding of a correct step): the CUDA path may not be further away than
+    # that (x1.5 + 0.03), and never further than 8e-2.
+    worst = ("", 0.0, 0.0)
+    errs, oerrs = [], []
+    for k in student:
+        gref = grads.get(k)
+        if gref is None or gref.norm().item() < 1e-9:
+            continue
+        e = (m.s_arena.g(k).float().cpu() - gref).norm().item() / gref.norm().item()
+        eo = (ostudent[k].grad - gref).norm().item() / gref.norm().item()
+        errs.append(e); oerrs.append(eo)
+        if e - 1.5 * eo > worst[1] - 1.5 * worst[2]:
+            worst = (k, e, eo)
+    rec["grad_rel_err"] = {"worst_excess": worst, "median": sorted(errs)[len(errs) // 2], "max": max(errs),
+                           "autocast_oracle_median": sorted(oerrs)[len(oerrs) // 2], "autocast_oracle_max": max(oerrs)}
+    assert worst[1] < 1.5 * worst[2] + 0.03, (worst, rec["grad_rel_err"])
+    assert rec["grad_rel_err"]["max"] < 8e-2, rec["grad_rel_err"]
+    assert rec["grad_rel_err"]["median"] < 1.5 * rec["grad_rel_err"]["autocast_oracle_median"] + 0.01, rec["grad_rel_err"]
     print("PARITY", rec)
     RESULTS[case.name] = rec
 

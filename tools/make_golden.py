@@ -1,8 +1,8 @@
-"""Generate tests/golden/* by running the REFERENCE's own modules (imported in place from /root/reference via
-oracle/ref_shim.py) on seeded inputs.  Runs in the build container only; the fixtures it writes are committed
-and are what the oracle (and through it the CUDA path) is pinned against on the GPU box.
+"""Generate tests/golden/* by running the REFERENCE's own modules (imported in place from a lightly-train source tree
+via oracle/ref_shim.py) on seeded inputs.  The fixtures it writes are committed and are what the oracle (and through it
+the CUDA path) is pinned against; the tests themselves never need the reference.
 
-    python tools/make_golden.py
+    LIGHTLY_TRAIN_SRC=<lightly-train checkout>/src python tools/make_golden.py
 
 Glue that cannot be imported (the LightningModule shell, LT/_methods/dinov2/dinov2.py:259-519, needs
 pytorch_lightning/lightly) is composed here from the reference's modules in the same order; KoLeoLoss
