@@ -22,43 +22,6 @@ def rnd(*shape, scale=1.0, dtype=torch.float32, seed=None):
     return (torch.randn(*shape, generator=g) * scale).to(dev).to(dtype)
 
 
-@pytest.mark.parametrize("M,N,K,a_mn,b_mn", [(256, 384, 128, 0, 0), (1000, 1152, 384, 0, 0), (384, 1152, 1000, 1, 1),
-                                             (300, 256, 520, 0, 1), (136, 392, 72, 1, 0)])
-def test_gemm_plain(M, N, K, a_mn, b_mn):
-    a = rnd(*((K, M) if a_mn else (M, K)), dtype=torch.bfloat16, seed=1)
-    b = rnd(*((K, N) if b_mn else (N, K)), dtype=torch.bfloat16, seed=2)
-    out = torch.empty(M, N, device=dev)
-    ops.gemm(a, b, out, a_mn=bool(a_mn), b_mn=bool(b_mn), epi=ops.EPI_F32)
-    A = a.float().t() if a_mn else a.float()
-    Bm = b.float().t() if b_mn else b.float()
-    torch.testing.assert_close(out, A @ Bm.t(), rtol=1e-4, atol=1e-3)
-
-
-@pytest.mark.parametrize("M,N,K,a_mn,b_mn,bn", [(1000, 1152, 384, 0, 0, 192), (1100, 392, 72, 0, 0, 128),
-                                                 (384, 1152, 1000, 1, 1, 256), (512, 256, 128, 1, 0, 128),
-                                                 (18944, 1152, 384, 0, 0, 0)])
-def test_gemm_cta_pair_kernel(M, N, K, a_mn, b_mn, bn):
-    """cta_group::2 schedule (256-row tiles, B split across the CTA pair): forced with ws_mode=3, and the shape the auto
-    heuristic routes to it (bn=0: M = 148 x 128 rows, plain epilogue)."""
-    a = rnd(*((K, M) if a_mn else (M, K)), dtype=torch.bfloat16, seed=1)
-    b = rnd(*((K, N) if b_mn else (N, K)), dtype=torch.bfloat16, seed=2)
-    out = torch.empty(M, N, device=dev)
-    ops.gemm(a, b, out, a_mn=bool(a_mn), b_mn=bool(b_mn), epi=ops.EPI_F32, block_n=bn, ws_mode=3 if bn else 0)
-    A = a.float().t() if a_mn else a.float()
-    Bm = b.float().t() if b_mn else b.float()
-    torch.testing.assert_close(out, A @ Bm.t(), rtol=1e-4, atol=1e-3)
-    # split-K accumulation and a fused epilogue through the pair kernel
-    if not a_mn and not b_mn and bn:
-        acc = torch.ones(M, N, device=dev)
-        ops.gemm(a, b, acc, epi=ops.EPI_F32_ATOMIC, splits=3, block_n=bn, ws_mode=3)
-        torch.testing.assert_close(acc, A @ Bm.t() + 1, rtol=1e-4, atol=2e-3)
-        bias, gamma, x = rnd(N, seed=5), rnd(N, seed=6), rnd(M, N, seed=7)
-        o2 = torch.empty(M, N, device=dev, dtype=torch.bfloat16)
-        ops.gemm(a, b, out, epi=ops.EPI_RESIDUAL, bias=bias, out2=o2, aux=x, gamma=gamma, block_n=bn, ws_mode=3)
-        torch.testing.assert_close(out, x + o2.float() * gamma, rtol=1e-5, atol=1e-5)
-        torch.testing.assert_close(o2.float(), (A @ Bm.t() + bias).bfloat16().float(), rtol=2e-2, atol=2e-2)
-
-
 def test_gemm_fused_epilogues():
     M, N, K = 777, 384, 1536
     a, b = rnd(M, K, dtype=torch.bfloat16, scale=0.5, seed=3), rnd(N, K, dtype=torch.bfloat16, scale=0.05, seed=4)
@@ -100,14 +63,6 @@ def test_gemm_saved_derivative_gelu_epilogues():
     ops.gemm(dy, w, dU, b_mn=True, epi=ops.EPI_MUL_AUX, aux=g)
     want = (dy.float() @ w.float()).bfloat16().float() * g.float()
     torch.testing.assert_close(dU.float(), want.bfloat16().float(), rtol=2e-2, atol=2e-2)
-
-
-def test_gemm_splitk_atomic_accumulates():
-    M, N, K = 1152, 384, 9000
-    a, b = rnd(K, M, dtype=torch.bfloat16, seed=8), rnd(K, N, dtype=torch.bfloat16, seed=9)
-    out = torch.ones(M, N, device=dev)
-    ops.gemm(a, b, out, a_mn=True, b_mn=True, epi=ops.EPI_F32_ATOMIC, splits=13)
-    torch.testing.assert_close(out, 1 + a.float().t() @ b.float(), rtol=1e-4, atol=2e-2)
 
 
 @pytest.mark.parametrize("B,N,h", [(3, 197, 6), (5, 37, 2), (2, 261, 3), (2, 54, 2), (1, 16, 1)])
